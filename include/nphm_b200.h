@@ -231,6 +231,26 @@ int nphm_mlp_backward_inputs(nphm_mlp *h, const float *xyz_dev, const float *con
 int nphm_mlp_inverse_jacobian(nphm_mlp *h, const float *xyz_dev, const float *cond_dev, int n_queries, long long n_points,
                               float *out_dev, float *jinv_dev, void *stream);
 
+/* First-order training of a layer-chain stack (the deformation network of stage-2 training, reference
+ * scripts/training/train_corresp.py).  The condition of query q at point n is cond_q + (noise_qn, 0): noise_dev
+ * [q][n][noise_dim] is added to the first noise_dim condition columns (noise_dim 0: none; at most 36).
+ * nphm_mlp_train_workspace_bytes: size of the device workspace one training forward needs (-1 on bad arguments). */
+long long nphm_mlp_train_workspace_bytes(const nphm_mlp *h, int n_queries, long long n_points, int noise_dim);
+/* == DeepSDF.forward on [xyz | cond_q + (noise_qn, 0)]: out_dev [q][n][out_dim]; keeps what the backward needs in workspace_dev */
+int nphm_mlp_forward_train(nphm_mlp *h, const float *xyz_dev, const float *cond_dev, const float *noise_dev, int noise_dim,
+                           int n_queries, long long n_points, float *out_dev, void *workspace_dev, void *stream);
+/* Gradients of sum(out * grad_out) for the forward held in workspace_dev (same arguments): grad_w_dev[l] [N_l][in_l] and
+ * grad_b_dev[l] [N_l] in the state_dict layout (condition columns included), grad_cond_dev [q][cond_dim], grad_xyz_dev [q][n][3].
+ * Every output may be NULL (grad_w_dev == NULL: no weight GEMMs; a NULL entry skips that layer); outputs are overwritten, not
+ * accumulated, and the weight gradients are bitwise reproducible.  A workspace of another shape, another handle or of weights
+ * loaded before the forward is refused with NPHM_ERR_INVALID, and so is a result that is not finite (an adjoint beyond the fp16
+ * range of the packed activation format, or non-finite weights / inputs).  Synchronises the stream twice: to read the workspace
+ * header and the scale of grad_out, and to check the outputs. */
+int nphm_mlp_backward_train(nphm_mlp *h, const float *xyz_dev, const float *cond_dev, const float *noise_dev, int noise_dim,
+                            int n_queries, long long n_points, const float *grad_out_dev, float *const *grad_w_dev,
+                            float *const *grad_b_dev, float *grad_cond_dev, float *grad_xyz_dev, void *workspace_dev,
+                            void *stream);
+
 /* anchors_dev [n_queries][n_loc][3] = mlp_pos(z_glob) + mean anchors (reference src/NPHM/models/EnsembledDeepSDF.py:228-229)
  * without evaluating the ensemble - what the fitters read from `decoder(zeros(1,1,3), lat)[1]` (fitting.py:59, :211). */
 int nphm_ensemble_anchors(nphm_ensemble *h, const float *latents_dev, int n_queries, float *anchors_dev, void *stream);

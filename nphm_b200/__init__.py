@@ -29,6 +29,21 @@ def _os_path_join(*a):
     return os.path.join(*a)
 
 
+def set_native_training(enabled: bool = True) -> None:
+    """Run first-order training through the native kernels: a ``DeepSDF`` / ``DeformationNetwork`` forward that autograd
+    records (and that the layer chain supports) then runs on sm_100a, and its backward computes the weight gradients there.
+    Default off, or on with the environment variable ``NPHM_NATIVE_TRAINING=1``.  Leave it off for losses that differentiate
+    twice (stage-1 identity training): the native backward is first order and raises under ``create_graph=True``."""
+    from . import _native
+    _native.set_native_training(enabled)
+
+
+def native_training() -> bool:
+    """Whether :func:`set_native_training` is on."""
+    from . import _native
+    return _native.native_training()
+
+
 def install_as_nphm(force: bool = False):
     """Register this package's mirrors under the reference's import names, so that
     ``from NPHM.models.deepSDF import DeepSDF`` (and the six other hot-path modules) resolve here, while every OTHER

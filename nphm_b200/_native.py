@@ -33,11 +33,28 @@ EXPORTED_SYMBOLS = (
     'nphm_fit_workspace_bytes', 'nphm_fit_identity_step', 'nphm_fit_surface_grad', 'nphm_fit_apply_gradient',
     'nphm_ensemble_backward_inputs', 'nphm_ensemble_anchors',
     'nphm_broyden_workspace_bytes', 'nphm_mlp_broyden_search', 'nphm_nearest_neighbors',
+    'nphm_mlp_train_workspace_bytes', 'nphm_mlp_forward_train', 'nphm_mlp_backward_train',
 )
 
 
 class NativeError(RuntimeError):
     pass
+
+
+# Native first-order training (DeepSDF / DeformationNetwork forwards recorded by autograd run on the layer chain and its
+# weight-gradient GEMMs).  Opt-in: at forward time it cannot be seen whether a double backward will follow, and the identity
+# losses (stage 1) differentiate the spatial gradient through the same forward.
+_native_training = os.environ.get('NPHM_NATIVE_TRAINING', '0') == '1'
+
+
+def set_native_training(enabled: bool = True) -> None:
+    """Switch native first-order training on or off (initial value: environment variable ``NPHM_NATIVE_TRAINING=1``)."""
+    global _native_training
+    _native_training = bool(enabled)
+
+
+def native_training() -> bool:
+    return _native_training
 
 
 # kernels of this library launched per call (ncu launch lists under profiles/); bench.py counts its launches with these
@@ -149,6 +166,12 @@ def lib() -> ctypes.CDLL:
                                           c_float, c_float, c_float, c_void_p, c_void_p, POINTER(c_int), c_void_p,
                                           c_void_p]
     L.nphm_nearest_neighbors.argtypes = [c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_void_p, c_void_p]
+    L.nphm_mlp_train_workspace_bytes.argtypes = [c_void_p, c_int, c_longlong, c_int]
+    L.nphm_mlp_train_workspace_bytes.restype = c_longlong
+    L.nphm_mlp_forward_train.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_longlong, c_void_p, c_void_p,
+                                         c_void_p]
+    L.nphm_mlp_backward_train.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_longlong, c_void_p,
+                                          POINTER(c_void_p), POINTER(c_void_p), c_void_p, c_void_p, c_void_p, c_void_p]
     for name in EXPORTED_SYMBOLS:                      # fail at load time, not at first use, if a symbol is missing
         getattr(L, name)
     _lib = L
@@ -353,6 +376,7 @@ class MlpEngine(_Versioned):
         # (csrc/tc_linear.cu, any width - e.g. the NPM baseline 515 -> 1024 x 8); the fp32 FFMA kernel is kept for impl='simt'
         self.fused_shape = (hidden == 512 and self.n_lin == 7 and module.lat_dim == 232 and module.out_dim_net == 3)
         self.simt_ok = hidden <= 880
+        self.shapes = [tuple(getattr(module, 'lin%d' % i).weight.shape) for i in range(self.n_lin)]
         self._sig = None
 
     def __del__(self):
@@ -449,6 +473,58 @@ class MlpEngine(_Versioned):
                                                  g.data_ptr(), g_cond.data_ptr(), _ptr(g_xyz), _stream_ptr(dev)),
                   'nphm_mlp_backward_inputs')
         return g_cond, g_xyz
+
+    def forward_train(self, xyz: torch.Tensor, cond: torch.Tensor, noise: Optional[torch.Tensor] = None):
+        """Training forward (nphm_mlp_forward_train): xyz B x N x 3, cond B x lat_dim, noise B x N x noise_dim (added to the
+        first noise_dim condition columns) or None -> (out B x N x out_dim, workspace).  The workspace (a uint8 tensor allocated
+        on the current stream) holds the activations ``backward_train`` reads."""
+        B, N, _ = xyz.shape
+        dev = xyz.device
+        xyz = _f32c(xyz)
+        cond = _f32c(cond).to(dev)
+        nd = 0 if noise is None else int(noise.shape[-1])
+        noise = None if noise is None else _f32c(noise)
+        out = torch.empty(B, N, self.out_dim, device=dev, dtype=torch.float32)
+        with torch.cuda.device(dev):
+            n_bytes = int(lib().nphm_mlp_train_workspace_bytes(self._h, B, N, nd))
+            if n_bytes < 0:
+                check(-1, 'nphm_mlp_train_workspace_bytes')
+            ws = torch.empty(n_bytes, device=dev, dtype=torch.uint8)
+            check(lib().nphm_mlp_forward_train(self._h, xyz.data_ptr(), cond.data_ptr(), _ptr(noise), nd, B, N, out.data_ptr(),
+                                               ws.data_ptr(), _stream_ptr(dev)), 'nphm_mlp_forward_train')
+        return out, ws
+
+    def backward_train(self, xyz: torch.Tensor, cond: torch.Tensor, noise: Optional[torch.Tensor], workspace: torch.Tensor,
+                       grad_out: torch.Tensor, want_w=True, want_b=True, want_cond: bool = True, want_xyz: bool = True):
+        """Gradients of ``sum(out * grad_out)`` for the ``forward_train`` call that filled ``workspace`` (nphm_mlp_backward_train).
+        ``want_w`` / ``want_b``: bool, or one bool per layer.  Returns (grad_w list, grad_b list, d/d cond B x lat_dim,
+        d/d xyz B x N x 3); entries not asked for are None."""
+        B, N, _ = xyz.shape
+        dev = xyz.device
+        xyz = _f32c(xyz)
+        cond = _f32c(cond).to(dev)
+        nd = 0 if noise is None else int(noise.shape[-1])
+        noise = None if noise is None else _f32c(noise)
+        g = _f32c(grad_out)
+        per_layer = lambda want: [bool(want)] * self.n_lin if isinstance(want, bool) else [bool(w) for w in want]
+        ww, wb = per_layer(want_w), per_layer(want_b)
+        gw = [torch.empty(self.shapes[l], device=dev, dtype=torch.float32) if ww[l] else None for l in range(self.n_lin)]
+        gb = [torch.empty(self.shapes[l][0], device=dev, dtype=torch.float32) if wb[l] else None for l in range(self.n_lin)]
+        g_cond = torch.empty(B, cond.shape[-1], device=dev, dtype=torch.float32) if want_cond else None
+        g_xyz = torch.empty(B, N, 3, device=dev, dtype=torch.float32) if want_xyz else None
+
+        def ptrs(ts):
+            if not any(t is not None for t in ts):
+                return None
+            arr = (c_void_p * len(ts))()
+            for i, t in enumerate(ts):
+                arr[i] = None if t is None else t.data_ptr()
+            return arr
+        with torch.cuda.device(dev):
+            check(lib().nphm_mlp_backward_train(self._h, xyz.data_ptr(), cond.data_ptr(), _ptr(noise), nd, B, N, g.data_ptr(),
+                                                ptrs(gw), ptrs(gb), _ptr(g_cond), _ptr(g_xyz), workspace.data_ptr(),
+                                                _stream_ptr(dev)), 'nphm_mlp_backward_train')
+        return gw, gb, g_cond, g_xyz
 
     def broyden_search(self, obs: torch.Tensor, cond: torch.Tensor, x_init: torch.Tensor, J_inv_init: torch.Tensor,
                        max_steps: int = 15, cvg_thresh: float = 1e-6, dvg_thresh: float = 0.2, eps: float = 1e-6,

@@ -328,6 +328,7 @@ extern "C" int nphm_mlp_load_weights(nphm_mlp *h, const float *const *w_dev, con
     NPHM_REQUIRE(h && w_dev && b_dev, "nphm_mlp_load_weights: NULL argument");
     int rc = h->weights.load(h->dims, 1, w_dev, b_dev, static_cast<cudaStream_t>(stream_));
     if (rc) return rc;
+    ++h->weight_gen;
     fill_descriptors(h->dims, h->weights, 1, 0, h->cfg.lat_dim, 0, 0, h->net, h->spec);
     rc = tc_mlp_pack(h, static_cast<cudaStream_t>(stream_));
     if (rc) return rc;

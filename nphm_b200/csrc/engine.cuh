@@ -76,6 +76,7 @@ struct nphm_mlp {
                                     // kernel are still those of this condition, do not rebuild them
     // layer-by-layer tensor-core passes: any width, Jacobian, adjoint (mlp_chain.cu)
     nphm::MlpChain *chain = nullptr;
+    unsigned long long weight_gen = 0;   // bumped by every nphm_mlp_load_weights: training workspaces of older weights are refused
 };
 
 namespace nphm {

@@ -55,4 +55,26 @@ struct PackedLinear {
 int launch_linear(const PackedLinear &w, LinearParams p, cudaStream_t stream);
 
 }  // namespace tcl
+
+// Weight gradients over the rows of a batch (tc_wgrad.cu).  Deterministic: per-row-range partials in `scratch`, summed in order.
+// `bad` (optional, device): set to non-zero when a written output is not finite.
+namespace wg {
+// dst[n][k] = scale * sum_r D[r][n] A[r][k], n < N, k < K; D and A packed (tcgen05)
+int packed_packed(const uint8_t *D, int d_ksteps, int N, const uint8_t *A, int a_ksteps, int K, long long M, float scale, float *dst,
+                  int ld_dst, DeviceBuffer &scratch, unsigned int *bad, cudaStream_t stream);
+// skinny products, SIMT: dst_w[p][w] (transpose: dst_w[w][p]) = scale * sum_r P[r][p] R[r][w], w < Wr (P packed, R row-major);
+// dst_ones[p] = scale * sum_r P[r][p] (optional)
+int packed_rows(const uint8_t *P, int p_ksteps, int Pw, const float *R, int ldr, int Wr, long long M, float scale, float *dst_w, int ld_w,
+                bool transpose, float *dst_ones, DeviceBuffer &scratch, unsigned int *bad, cudaStream_t stream);
+// out[range][p] = sum of P[r][p] over the rows of each range of rows_per_range rows (P packed), fixed order
+int range_sums(const uint8_t *P, int p_ksteps, int Pw, long long M, long long rows_per_range, float *out, cudaStream_t stream);
+// *out_dev = bit pattern of max |x|;  y = s * x
+int abs_max(const float *x, long long n, unsigned int *out_dev, cudaStream_t stream);
+int scale(const float *x, long long n, float s, float *y, unsigned int *bad, cudaStream_t stream);
+// out[w] = sum_r R[r][w]  (R row-major)
+int rows_column_sums(const float *R, int ldr, int W, long long M, float *out, cudaStream_t stream);
+// dst[n][col0 + j] = scale * sum_q S[q][n] cond[q][j]  (added to what is there for j < n_add)
+int cond_columns(const float *S, int N, const float *cond, int cond_dim, int Q, float scale, int n_add, float *dst, int ld, int col0,
+                 unsigned int *bad, cudaStream_t stream);
+}  // namespace wg
 }  // namespace nphm

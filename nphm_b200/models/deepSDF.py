@@ -8,7 +8,9 @@ Reference interface (file:line):
 Parameter names (``lin{i}.weight/bias``, ``compressor.0.*``, ``defDeepSDF.lin{i}.*``) and
 constructor signatures are those of the reference so checkpoints load with ``strict=True``.
 As in :mod:`.EnsembledDeepSDF`, CUDA no-grad calls with a per-query-constant condition run in
-the native sm_100a MLP kernel; everything else uses a PyTorch composite that keeps autograd.
+the native sm_100a MLP kernel.  With :func:`nphm_b200.set_native_training` on, forwards that autograd
+records run natively as well (:class:`_NativeTrain`: first order only); everything else uses a
+PyTorch composite that keeps autograd.
 """
 from __future__ import annotations
 
@@ -18,12 +20,54 @@ from typing import Optional
 import numpy as np
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from .. import _native
 from . import _composite
 from .EnsembledDeepSDF import sample_point_feature  # same function in the reference (:92-115)
 
 _SQRT2 = math.sqrt(2.0)
+
+
+def condition_noise(shape, device) -> torch.Tensor:
+    """Training-mode noise on the compressed identity code (reference deepSDF.py:220-221).  Both the composite and the
+    native path draw it here, with the same call, so that seeded runs of either see the same numbers."""
+    return torch.randn(shape, device=device) / 200
+
+
+class _NativeTrain(torch.autograd.Function):
+    """Backbone forward on [xyz | cond_q + (noise, 0)] with native first-order backward (nphm_mlp_forward_train /
+    nphm_mlp_backward_train).  Inputs: backbone module, xyz B x N x 3, per-query condition B x lat_dim, noise B x N x k or None,
+    then the weights and biases of every layer (saved, so that an in-place change before the backward is caught)."""
+
+    @staticmethod
+    def forward(ctx, backbone, xyz, cond, noise, *params):
+        eng = backbone.engine()
+        out, ws = eng.forward_train(xyz, cond, noise)
+        ctx.eng, ctx.ws, ctx.noise = eng, ws, noise
+        ctx.save_for_backward(xyz, cond, *params)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        if torch.is_grad_enabled():
+            raise RuntimeError('the native training backward is first order only (create_graph=True asks for more): switch it '
+                               'off with nphm_b200.set_native_training(False) for losses that differentiate twice')
+        return _native_train_backward(ctx, grad_out)
+
+
+@once_differentiable
+def _native_train_backward(ctx, grad_out):
+    if ctx.ws is None:
+        raise RuntimeError('a native training forward can be differentiated once: its workspace is released by the first '
+                           'backward (retain_graph=True is not supported with nphm_b200.set_native_training(True))')
+    xyz, cond, *params = ctx.saved_tensors             # raises if a weight was modified in place since the forward
+    need = ctx.needs_input_grad
+    gw, gb, g_cond, g_xyz = ctx.eng.backward_train(xyz, cond, ctx.noise, ctx.ws, grad_out, want_w=need[4::2],
+                                                   want_b=need[5::2], want_cond=need[2], want_xyz=need[1])
+    ctx.ws = None                                      # the workspace (activations of the whole batch) goes with the first backward
+    grads = [g for pair in zip(gw, gb) for g in pair]
+    return (None, g_xyz, g_cond, None, *grads)
 
 
 class DeepSDF(nn.Module):
@@ -86,7 +130,37 @@ class DeepSDF(nn.Module):
             return False
         return xyz.dtype == torch.float32 and xyz.dim() == 3
 
+    def _native_train_ok(self, xyz, lat_rep) -> bool:
+        """A training forward (autograd recording, something requires grad) the native path takes; the condition must still
+        be constant per query (checked by the caller)."""
+        if not _native.native_training() or not torch.is_grad_enabled():
+            return False
+        if not (xyz.requires_grad or lat_rep.requires_grad or any(p.requires_grad for p in self.parameters())):
+            return False
+        if not (xyz.is_cuda and lat_rep.is_cuda and xyz.dtype == torch.float32 and lat_rep.dtype == torch.float32
+                and xyz.dim() == 3 and xyz.shape[-1] == 3 and xyz.shape[1] > 0 and lat_rep.dim() == 3
+                and lat_rep.shape[0] == xyz.shape[0]):
+            return False
+        if self.num_freq_bands is not None or self.beta != 100 or self.out_dim_net > 8:
+            return False
+        n_lin = self.num_layers - 1
+        if not _native.stack_supported(n_lin - 1, _native.hidden_width(self, n_lin), self.lat_dim):
+            return False
+        return 1 <= self.skip_in[0] < n_lin - 1           # chain_ready's skip constraint (csrc/mlp_chain.cu)
+
+    def forward_native_train(self, xyz, cond, noise=None):
+        """xyz B x N x 3, cond B x lat_dim (per query), noise B x N x k or None -> B x N x out_dim, native backward."""
+        params = []
+        for i in range(self.num_layers - 1):
+            lin = getattr(self, 'lin%d' % i)
+            params += [lin.weight, lin.bias]
+        return _NativeTrain.apply(self, xyz, cond, noise, *params)
+
     def forward(self, xyz, lat_rep, anchors=None):
+        if self._native_train_ok(xyz, lat_rep):
+            cond = _native.constant_latent_rows(lat_rep)
+            if cond is not None:
+                return self.forward_native_train(xyz, cond), None
         if self._fused_ok(xyz, lat_rep):
             cond = _native.constant_latent_rows(lat_rep)
             if cond is not None:
@@ -196,9 +270,10 @@ class DeformationNetwork(nn.Module):
         self.anchors = anchors
 
     # ------------------------------------------------------------------
-    def _condition(self, xyz, lat_rep, anchors, per_point: bool):
+    def _condition(self, xyz, lat_rep, anchors, per_point: bool, with_noise: bool = True):
         """Condition vector of the backbone.  ``per_point=False`` returns ``B x 1 x C`` when the
-        mode allows a per-query constant (used by the fused path)."""
+        mode allows a per-query constant (used by the fused path; ``with_noise=False``: also in training
+        mode, the native training path adds the noise itself)."""
         B, N, _ = xyz.shape
         E = self.lat_dim_expr
         if self.mode == 'glob_only':
@@ -217,10 +292,10 @@ class DeformationNetwork(nn.Module):
             a0 = anchors[:, 0] if anchors.dim() == 4 else anchors                 # B x K x 3
             first = torch.cat([lat_rep[:, 0, :-E], a0.reshape(B, -1)], dim=-1)     # B x 1461
             compressed = self.compressor(first).unsqueeze(1)                      # B x 1 x 32
-            if per_point or self.training:
+            if per_point or (self.training and with_noise):
                 compressed = compressed.expand(B, N, compressed.shape[-1])
-                if self.training:
-                    compressed = compressed + torch.randn(compressed.shape, device=compressed.device) / 200
+                if self.training and with_noise:
+                    compressed = compressed + condition_noise(compressed.shape, compressed.device)
                 return torch.cat([compressed, lat_rep[..., -E:].expand(B, N, E)], dim=-1)
             return torch.cat([compressed, lat_rep[:, :1, -E:]], dim=-1)           # B x 1 x 232
         if self.mode == 'GNN':
@@ -255,6 +330,16 @@ class DeformationNetwork(nn.Module):
         if xyz.dim() < 3:
             xyz = xyz.unsqueeze(0)
         backbone = self.defDeepSDF
+        if self.mode in ('compress', 'expr_only', 'glob_only') and backbone._native_train_ok(xyz, lat_rep):
+            lat = _native.constant_latent_rows(lat_rep)
+            if lat is not None:
+                # condition built in torch (compressor, anchors upstream keep autograd); the noise rides with xyz
+                B, N, _ = xyz.shape
+                cond = self._condition(xyz, lat.unsqueeze(1), anchors, per_point=False, with_noise=False)[:, 0]
+                noise = (condition_noise((B, N, self.compressor[0].out_features), xyz.device)
+                         if self.training and self.mode == 'compress' else None)
+                pred = backbone.forward_native_train(xyz, cond, noise)
+                return pred[..., :3], pred[..., -1:]
         fused = (backbone._fused_ok(xyz, lat_rep) and not self.training
                  and self.mode in ('compress', 'expr_only', 'glob_only')
                  and not (anchors is not None and torch.is_grad_enabled() and anchors.requires_grad))

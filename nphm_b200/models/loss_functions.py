@@ -2,6 +2,7 @@
 
   * ``compute_loss``         src/NPHM/models/loss_functions.py:7-17
   * ``actual_compute_loss``  src/NPHM/models/loss_functions.py:20-110   (SURVEY.md 8f-3)
+  * ``compute_loss_corresp_forward``  src/NPHM/models/loss_functions.py:282-322  (stage-2 expression training)
 
 Same inputs (a batch dict with ``points_face``, ``points_non_face``, ``sup_grad_far``, ``sup_grad_near``, the normals and
 ``gt_anchors``), same returned dict (``surf_sdf``, ``normals``, ``space_sdf``, ``grad``, ``lat_reg`` and - for the
@@ -110,3 +111,30 @@ def actual_compute_loss(batch_cuda, decoder, glob_cond, native=None):
     losses['symm_dist'] = symm_dist
     losses['middle_dist'] = middle_dist
     return losses
+
+
+def compute_loss_corresp_forward(batch, decoder, decoder_shape, latent_codes, latent_codes_shape, device, epoch=-1,
+                                 exp_path=None):
+    """Stage-2 training loss of the deformation network (same signature and returned dict as the reference): squared error of
+    the posed correspondences, the expression-code magnitude, and the deformation of 100 uniform samples per query in
+    [-1.25, 1.25)^3 pushed towards zero.  ``epoch`` and ``exp_path`` are unused, as in the reference.  Both decoder calls
+    see a per-query-constant condition, so with :func:`nphm_b200.set_native_training` on they run natively."""
+    batch.pop('path', None)
+    on_device = {k: v.to(device).float() for k, v in batch.items()}
+    cond_shape = latent_codes_shape(batch['subj_ind'].to(device))
+    cond_pose = latent_codes(batch['idx'].to(device))
+    if decoder_shape is not None and decoder_shape.mlp_pos is not None:
+        anchors = decoder_shape.mlp_pos(cond_shape[..., :decoder_shape.lat_dim_glob]).view(cond_pose.shape[0], -1, 3)
+        anchors += decoder.anchors.squeeze(0)
+    else:
+        anchors = on_device['gt_anchors']
+    glob_cond = torch.cat([cond_shape, cond_pose], dim=-1)
+    points = on_device['points_neutral'].clone().detach().requires_grad_()
+    cond = glob_cond.repeat(1, points.shape[1], 1)
+    delta, _ = decoder(points, cond, anchors)
+    corresp = (points + delta.squeeze() - on_device['points_posed'][:, :, :3]) ** 2
+    samples = (torch.rand(cond.shape[0], 100, 3, device=cond.device, dtype=cond.dtype) - 0.5) * 2.5
+    delta_samples, _ = decoder(samples, cond[:, :100, :], anchors)
+    return {'corresp': corresp.mean(),
+            'lat_reg': (torch.norm(cond_pose, dim=-1) ** 2).mean(),
+            'loss_reg_zero': (delta_samples ** 2).mean()}
